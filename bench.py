@@ -7,6 +7,7 @@ ppo_update kernels.  A "step" is one iteration = 128 vec-env steps + critic pass
 = 4096*128 env-steps per GPU.
 
     python bench.py --gpus 1 --steps 10 --warmup 3
+    python bench.py --gpus 1 --steps 10 --warmup 3 --dump-outputs DIR   # + the last timed iteration's outputs, DIR/*.npy
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...
     python bench.py --impl reference          # CPU restatement of the reference path (oracle port)
 
@@ -195,11 +196,42 @@ def gae_roofline(flush, steps=10):
     return out
 
 
-def time_iterations(drv, steps, warmup, flush, world):
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def iteration_outputs(drv):
+    """What one `device_iteration` hands its caller, as host arrays: the rollout buffer it filled (observations, actions,
+    log-probs, rewards, masks, value predictions, returns, advantages), the updated policy / critic parameters, the
+    ValueNorm state and the six per-update means of the logged loss terms (`train_info`, as `read_train_info` forms them);
+    all float32."""
+    d, tr = drv.buffer.data, drv.trainer
+    out = {name: getattr(d, name) for name in ("policy_obs", "actions", "action_log_probs", "rewards", "masks", "active_masks",
+                                               "value_preds", "returns", "advantages")}
+    out["policy_params"] = tr.algo_module.models["policy"].flat_params
+    out["critic_params"] = tr.algo_module.models["critic"].flat_params
+    out["value_norm_state"] = tr.algo_module.get_critic_value_normalizer().state
+    out["train_info"] = tr.train_info / (tr.ppo_epoch * tr.num_mini_batch)
+    out = {k: v.detach().float().cpu().numpy() for k, v in out.items()}
+    total = sum(a.nbytes for a in out.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise RuntimeError(f"--dump-outputs: {total} bytes exceed the {DUMP_LIMIT_BYTES} byte limit")
+    return out
+
+
+def dump_outputs(outputs, directory):
+    import numpy as np
+
+    os.makedirs(directory, exist_ok=True)
+    for name, a in outputs.items():
+        np.save(os.path.join(directory, f"{name}.npy"), a)
+
+
+def time_iterations(drv, steps, warmup, flush, world, after_timed=None):
     """W untimed + K timed device iterations (collect + update) through `OnPolicyDriver.device_iteration` — one captured
     CUDA graph replay per iteration when eligible (the product's default), else ~25 launches — CUDA events per iteration
     on the launching stream, 256 MB L2 flush between timed iterations, max over ranks.  The per-phase times come from a
-    separate short eager pass (events cannot be read inside a graph).
+    separate short eager pass (events cannot be read inside a graph); `after_timed(drv)`, when given, runs between the
+    timed iterations and that pass, while the driver still holds what the last timed iteration computed.
     Returns (seconds, phases_ms, launches, wall window)."""
     import torch
     import torch.distributed as dist
@@ -227,6 +259,8 @@ def time_iterations(drv, steps, warmup, flush, world):
     window = (t0, time.time())
     launches = drv.gpu_launches + drv.trainer.gpu_launches - l0
     total_s = sum(a.elapsed_time(b) for a, b in events) * 1e-3
+    if after_timed is not None:
+        after_timed(drv)
     # phases: eager pass
     drv.phase_events = []
     for _ in range(3):
@@ -357,7 +391,10 @@ def run_ours(args):
     sampler = ClockSampler(local)
     if rank == 0:
         sampler.start()
-    total_s, phases, launches, window = time_iterations(drv, args.steps, args.warmup, flush, world)
+    dump = None
+    if args.dump_outputs and rank == 0:
+        dump = lambda d: dump_outputs(iteration_outputs(d), args.dump_outputs)  # noqa: E731
+    total_s, phases, launches, window = time_iterations(drv, args.steps, args.warmup, flush, world, after_timed=dump)
     sampler.window = window
     clocks = sampler.stop() if rank == 0 else None
     env_steps = N_ENVS * T * args.steps * world
@@ -494,7 +531,7 @@ def _best_cpu_threads(n_envs):
 
 
 def cpu_baseline_sample(n_envs=256, iters=1):
-    """cpu_baseline leg: the unmodified reference (`kind: reference`, baseline/_ref through
+    """cpu_baseline leg: the unmodified reference (`kind: reference`, oracle/_ref through
     oracle/run_reference.py, SyncVectorEnv, 128 of the 4096 envs, all host cores) with the oracle port
     (oracle/loop.py) timed beside it as a second, labelled number."""
     from oracle import loop as oloop
@@ -510,18 +547,18 @@ def cpu_baseline_sample(n_envs=256, iters=1):
     port = {"value": n_envs * T * iters / dt, "unit": "env-steps/s", "cores": threads, "kind": "port",
             "sample": f"{iters} iteration(s) of {n_envs} envs x T={T}, {EPOCHS} epochs (oracle/loop.py, torch-CPU + numpy)"}
     if not reference_available():
-        return {**port, "note": "baseline/_ref missing: port only"}
+        return {**port, "note": "oracle/_ref missing: port only"}
     try:
         ref = reference_run(REF_ENVS, 5, 3)
     except Exception as e:  # noqa: BLE001
         return {**port, "note": f"reference run failed ({str(e)[-200:]}): port only"}
     return {"value": ref["env_steps_per_s"], "unit": "env-steps/s", "cores": ref["torch_threads"], "kind": "reference",
             "sample": f"5 PPOAgent.train iterations (after 3 warm-up) of {REF_ENVS} of the {N_ENVS} envs x T={T}, {EPOCHS} epochs; unmodified "
-                      f"reference from baseline/_ref, SyncVectorEnv, {ref['host_cores']} host cores", "port": port}
+                      f"reference from oracle/_ref, SyncVectorEnv, {ref['host_cores']} host cores", "port": port}
 
 
 def reference_run(envs, iters, warmup, asynchronous=False, timeout=300):
-    """One timed run of the UNMODIFIED reference (baseline/_ref, oracle/run_reference.py) in a fresh
+    """One timed run of the UNMODIFIED reference (oracle/_ref, oracle/run_reference.py) in a fresh
     process: `PPOAgent.train` on the host cores, all of them (the child resets torchrun's OMP_NUM_THREADS=1)."""
     cmd = [sys.executable, os.path.join(ROOT, "oracle", "run_reference.py"), "--env", "CartPole-v1", "--envs", str(envs),
            "--T", str(T), "--epochs", str(EPOCHS), "--minibatch", str(MINIBATCH), "--iters", str(iters), "--warmup", str(warmup)]
@@ -536,7 +573,7 @@ def reference_run(envs, iters, warmup, asynchronous=False, timeout=300):
 
 
 def reference_available():
-    return os.path.isfile(os.path.join(ROOT, "baseline", "_ref", "openrl", "__init__.py"))
+    return os.path.isfile(os.path.join(ROOT, "oracle", "_ref", "openrl", "__init__.py"))
 
 
 REF_ENVS = 128   # north_star's target point; the reference's per-env Python loop makes cost linear in envs
@@ -569,7 +606,7 @@ def run_reference(args):
             extra["c1"] = {"error": str(e)[-300:]}
         extra["not_run"] = "AsyncVectorEnv at 4096 envs = 4097 processes: infeasible on this host; Sync at 4096 envs is ~30 s/iteration"
         cores, sample = sync["torch_threads"], (f"each step = one PPOAgent.train iteration of {REF_ENVS} of the {N_ENVS} envs x T={T}, {EPOCHS} epochs, "
-                                                 f"unmodified reference (baseline/_ref) + SyncVectorEnv, {sync['host_cores']} host cores")
+                                                 f"unmodified reference (oracle/_ref) + SyncVectorEnv, {sync['host_cores']} host cores")
         dt = sync["seconds"]
     else:
         from oracle import loop as oloop
@@ -584,7 +621,7 @@ def run_reference(args):
         for _ in range(steps):
             tr.iteration()
         dt = time.perf_counter() - t0
-        value, kind, cores, extra = n_envs * T * steps / dt, "port", threads, {"note": "baseline/_ref missing: oracle port timed instead"}
+        value, kind, cores, extra = n_envs * T * steps / dt, "port", threads, {"note": "oracle/_ref missing: oracle port timed instead"}
         sample = f"each step = one iteration of {n_envs} of the {N_ENVS} envs x T={T}, {EPOCHS} epochs (oracle/loop.py)"
     cb = {"value": value, "unit": "env-steps/s", "cores": cores, "kind": kind, "sample": sample}
     print(json.dumps({**base, "value": value, "ms_per_step": dt / steps * 1e3, "cpu_baseline": cb, "reference_runs": extra,
@@ -600,7 +637,11 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true", help="development: skip the cpu_baseline leg")
     ap.add_argument("--no-extras", action="store_true", help="skip the extras block (other configs / modes)")
     ap.add_argument("--only-extra", default="", help="development: comma-separated names of the extras to run")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="write what the last timed iteration computed (rank 0) as DIR/<name>.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be >= 1")
     if args.impl == "reference":
         run_reference(args)
     else:

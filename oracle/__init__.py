@@ -11,3 +11,7 @@ is pinned against outputs of the unmodified reference executed in the build cont
 CartPole-v1 dynamics come from third-party gymnasium (absent): that one boundary is
 "parity unpinned" (see oracle/cartpole_ref.py).
 """
+
+# Intra-op thread count the traces under tests/golden were recorded with.  MKL partitions its GEMM reductions and the QR
+# of `orthogonal_` by thread count, which moves last bits, so the bit-exact replays of those traces use the same count.
+TRACE_THREADS = 8

@@ -222,6 +222,10 @@ def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--only", default="")
     a = ap.parse_args()
+    sys.path.insert(0, os.path.dirname(HERE))
+    from oracle import TRACE_THREADS
+
+    torch.set_num_threads(TRACE_THREADS)
     os.makedirs(OUT, exist_ok=True)
     if a.only in ("", "gae"):
         gen_gae()

@@ -1,5 +1,5 @@
 #!/usr/bin/env python
-"""Time the UNMODIFIED reference (OpenRL, installed into baseline/_ref by oracle/make_ref.py) on the
+"""Time the UNMODIFIED reference (OpenRL, installed into oracle/_ref by oracle/make_ref.py) on the
 host cores: `PPOAgent.train` through the reference's own public API and stock code path.
 
 TEST / BENCH INFRASTRUCTURE (the reference arm of bench.py and the cpu_baseline leg).  Nothing of
@@ -22,13 +22,12 @@ import sys
 import time
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-ROOT = os.path.dirname(HERE)
 
 
 def ref_paths():
-    ref = os.path.join(ROOT, "baseline", "_ref")
+    ref = os.path.join(HERE, "_ref")
     if not os.path.isdir(os.path.join(ref, "openrl")):
-        raise SystemExit("baseline/_ref/openrl missing: run `python oracle/make_ref.py` in the build container")
+        raise SystemExit("oracle/_ref/openrl missing: run `python oracle/make_ref.py` where the reference source is")
     return [os.path.join(HERE, "refstubs"), HERE, ref]
 
 

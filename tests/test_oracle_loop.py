@@ -8,7 +8,16 @@ import pytest
 import torch
 
 from conftest import GOLDEN
-from oracle import loop
+from oracle import TRACE_THREADS, loop
+
+
+@pytest.fixture(autouse=True)
+def trace_threads():
+    """Replay with the thread count the traces were recorded with (bit-exact results depend on it)."""
+    prev = torch.get_num_threads()
+    torch.set_num_threads(TRACE_THREADS)
+    yield
+    torch.set_num_threads(prev)
 
 
 def _params(tr):
