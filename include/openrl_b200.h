@@ -230,6 +230,9 @@ int orl_policy_eval(const float* policy_params, int obs_dim, int n_actions, int 
 #define ORL_PPO_A2C 256               /* A2CAlgorithm.prepare_loss (openrl/algorithms/a2c.py:39-140): policy loss
                                          -adv * log-prob instead of the clipped surrogate; ratio reported as 0 */
 #define ORL_PPO_DUAL_CLIP 512         /* cfg.dual_clip_ppo: ratio = min(ratio, dual_clip_coeff) (ppo.py:304-305) */
+#define ORL_PPO_JOINT_ACTION 1024     /* cfg.use_joint_action_loss (JRPO, ppo.py:254-321): chunked recurrent update only
+                                         (orl_rnn_fwdbwd, n_agents <= 4); see the JRPO layout under OrlRnnArgs.  The
+                                         feed-forward entry points refuse it with ORL_ERR_UNSUPPORTED. */
 #define ORL_PPO_TENSORCORE 128        /* the 64x64 GEMMs of the trunk (forward, backward-data, weight gradients) on tcgen05
                                          tensor cores with split-fp16 operands (x = hi + lo, three MMA passes, FP32
                                          accumulate in TMEM): fp32-class accuracy, same 1e-4 loss-parity bar as the FFMA
@@ -338,6 +341,22 @@ int orl_minibatch_stats(const int64_t* indices, int64_t batch_rows, const float*
  * CPU against the oracle); parameter gradients are reductions of a per-row tape, dW = sum P^T Q.
  * Parameter layout of a recurrent net (reference state_dict order):
  *   W1[64][d] b1 g1 be1 | W3[64][64] b3 g3 be3 | Wih[192][64] Whh[192][64] bih bhh | g_rnn be_rnn | Wh[n][64] bh[n]
+ *
+ * JRPO (flags & ORL_PPO_JOINT_ACTION, cfg.use_joint_action_loss; ReplayData.recurrent_generator_v3
+ * replay_data.py:425-551, _cast_v3 / _flatten_v3 buffers/utils/util.py:92-101, PPOAlgorithm.prepare_loss
+ * ppo.py:222-224,254-321, ACTLayer.evaluate_actions act.py:114-118):
+ *   - chunks are per env: the flattening is g = n*T + t, every g carrying all A agents; chunk c covers
+ *     g in [c*L, c*L + L) (ignoring trajectory boundaries) and `chunk_ids` index these N*T / L chunks;
+ *   - policy: A sequences per chunk, agent a starting from rnn_states[t0][n0*A + a] (g0 = c*L = n0*T + t0);
+ *     per (chunk, step) the ratio is exp(sum_a logp_a - sum_a old_logp_a) (dual clip applies to it), the advantage
+ *     and, with ORL_PPO_POLICY_ACTIVE_MASKS, the row weight are agent 0's; every agent row of the step receives
+ *     the same dL/dlogp; the entropy is the mean over all agent rows (weighted by every agent's active mask with
+ *     ORL_PPO_POLICY_ACTIVE_MASKS);
+ *   - critic: agent 0 only (`to_single_np`): one sequence per chunk over rows n*A, n_chunks*L row-steps;
+ *   - mb_stats points to 4 doubles {sum ret_0, sum ret_0^2, sum active_0, sum active_all} over the minibatch
+ *     (agent 0's returns feed ValueNorm, ppo.py:190-191), norm_rows counts joint rows (chunk steps), the reported
+ *     ratio is the mean joint ratio;
+ *   - the tape holds n_chunks*L*A policy rows: size it with orl_rnn_workspace_floats(n_chunks*L*A, ...).
  */
 typedef struct OrlRnnArgs {
     int32_t env_kind, n_envs, n_agents, episode_length;   /* N, A, T; rows B = N*A */
@@ -358,7 +377,7 @@ typedef struct OrlRnnArgs {
     uint64_t rng_seed; uint64_t rng_step_base; uint64_t* rng_counter;
     double* env_f64; uint64_t* env_u64; int32_t* env_i32; const int32_t* env_table;
     float* ep_return; int32_t* ep_length; double* episode_stats;
-    const double* gae_stats; const double* mb_stats; float* vn_state;
+    const double* gae_stats; const double* mb_stats; float* vn_state;   /* mb_stats: 3 doubles (4 with ORL_PPO_JOINT_ACTION) */
     float* tape;                                          /* workspace: orl_rnn_workspace_floats(n_chunks*L, grads_stride) floats (tape rows, then reduction partials) */
     float* grads;                                         /* (2, grads_stride) true gradients, policy then critic */
     int32_t grads_stride; int32_t reserved1;
@@ -373,7 +392,8 @@ typedef struct OrlRnnArgs {
 } OrlRnnArgs;
 int orl_rnn_param_count(int obs_dim, int n_out);
 int orl_rnn_tape_width(void);
-/* floats of OrlRnnArgs.tape for a minibatch of `rows` = n_chunks * chunk_length row-steps */
+/* floats of OrlRnnArgs.tape for a minibatch of `rows` = n_chunks * chunk_length row-steps (times n_agents with
+   ORL_PPO_JOINT_ACTION) */
 long long orl_rnn_workspace_floats(long long rows, int grads_stride);
 /* policy GRU rollout for steps [t_begin, t_end) fused with the device env (simple_spread, CartPole, GridWorld) */
 int orl_rnn_rollout(const OrlRnnArgs* args, void* stream);

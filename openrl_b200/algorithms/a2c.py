@@ -7,6 +7,9 @@ from .ppo import PPOAlgorithm
 
 class A2CAlgorithm(PPOAlgorithm):
     def __init__(self, cfg, init_module, agent_num=1, device="cuda:0"):
+        if getattr(cfg, "use_joint_action_loss", False):
+            # the reference's A2C loss (a2c.py:39-140) has no joint-action branch
+            raise NotImplementedError("use_joint_action_loss with A2C is not built")
         super().__init__(cfg, init_module, agent_num, device)
         self.num_mini_batch = 1
         self.flags |= lib.PPO_A2C

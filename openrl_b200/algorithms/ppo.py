@@ -13,7 +13,7 @@ permutation is needed at all (a minibatch that is the whole buffer is a sum over
 import numpy as np
 import torch
 from .. import lib, parallel
-from ..buffers.replay_data import ReplayData, chunk_row_indices
+from ..buffers.replay_data import ReplayData, chunk_row_indices, chunk_row_indices_v3
 
 
 class PPOAlgorithm:
@@ -53,7 +53,7 @@ class PPOAlgorithm:
         self.grads = torch.zeros(2, self.grads_stride, dtype=torch.float32, device=dev)
         self.train_info = torch.zeros(6, dtype=torch.float32, device=dev)
         self.lrs = torch.zeros(2, dtype=torch.float32, device=dev)
-        self.mb_stats = torch.zeros(3, dtype=torch.float64, device=dev)
+        self.mb_stats = torch.zeros(4, dtype=torch.float64, device=dev)   # 3 doubles; the 4th is JRPO's all-agent active sum
         self.flags = ((lib.PPO_HUBER if cfg.use_huber_loss else 0) | (lib.PPO_CLIP_VALUE if cfg.use_clipped_value_loss else 0)
                       | (lib.PPO_VALUE_ACTIVE_MASKS if cfg.use_value_active_masks else 0)
                       | (lib.PPO_POLICY_ACTIVE_MASKS if cfg.use_policy_active_masks else 0)
@@ -67,6 +67,19 @@ class PPOAlgorithm:
         assert not (getattr(cfg, "use_popart", False) and cfg.use_valuenorm), \
             "self._use_popart and self._use_valuenorm can not be set True simultaneously"   # ppo.py:40-44
         self.share = bool(getattr(init_module, "share_model", False))
+        # JRPO (ppo.py:254-321, 363-369): the joint-action loss over recurrent_generator_v3 chunks; the reference takes it
+        # only with use_recurrent_policy
+        self.joint = bool(getattr(cfg, "use_joint_action_loss", False))
+        if self.joint:
+            if self.share or getattr(cfg, "use_share_model", False):
+                raise NotImplementedError("use_joint_action_loss with use_share_model is not built")
+            if self.naive:
+                raise NotImplementedError("use_joint_action_loss with use_naive_recurrent_policy is not built (the reference "
+                                          "applies the joint loss to naive_recurrent_generator batches of unrelated rows)")
+            if not cfg.use_recurrent_policy:
+                raise NotImplementedError("use_joint_action_loss needs use_recurrent_policy: with an MLP policy the reference's "
+                                          "feed_forward_generator groups agent_num random rows into one joint action")
+            self.flags |= lib.PPO_JOINT_ACTION
         if self.share:
             # one network, one optimiser: true-layout gradients + 8 loss-sum slots in ONE bucket (a single all-reduce per update)
             if self.recurrent:
@@ -78,8 +91,7 @@ class PPOAlgorithm:
             self.share_grads = self.share_bucket[:(self.share_total + 3) & ~3]
             self.share_loss = self.share_bucket[(self.share_total + 3) & ~3:]
             self.share_ws = None
-        for name in ("use_joint_action_loss", "use_policy_vhead",
-                     "use_amp", "use_deepspeed"):
+        for name in ("use_policy_vhead", "use_amp", "use_deepspeed"):
             if getattr(cfg, name, False):
                 raise NotImplementedError(f"cfg.{name} is not built into the CUDA update yet (SURVEY.md §8f)")
         if self.recurrent:
@@ -216,25 +228,44 @@ class PPOAlgorithm:
         a.norm_rows = rows * self.world_size if self.world_size > 1 else 0
         return a
 
+    def joint_minibatch_stats(self, buf, chunk_ids, chunk_length):
+        """JRPO minibatch moments {sum ret_0, sum ret_0^2, sum active_0, sum active_all} of the given v3 chunks into
+        self.mb_stats (this rank's rows only).  The all-agent pass writes slots 1..3 first, then the agent-0 pass
+        overwrites slots 0..2, so slot 3 keeps the all-agent active sum."""
+        s, T, N, A = lib.current_stream(), buf.episode_length, buf.n_rollout_threads, buf.num_agents
+        for agent0, out in ((False, self.mb_stats[1:]), (True, self.mb_stats)):
+            bi = chunk_row_indices_v3(chunk_ids, chunk_length, T, N, A, agent0_only=agent0)
+            lib.check(self._lib.orl_minibatch_stats(lib.ptr(bi), int(bi.numel()), lib.ptr(buf.returns),
+                                                    lib.ptr(buf.active_masks), lib.ptr(out), s), "orl_minibatch_stats")
+        self.gpu_launches += 2
+        return self.mb_stats
+
     def _train_recurrent(self, buf):
         """train_ppo with ReplayData.recurrent_generator (replay_data.py:1062-1258): per epoch one permutation of
         the data chunks (L consecutive steps of the agent-major / time-minor flattening f = (n*A + a)*T + t);
-        a minibatch is a slice of chunk ids, gathered inside the kernels."""
+        a minibatch is a slice of chunk ids, gathered inside the kernels.
+
+        With the joint-action loss (recurrent_generator_v3, replay_data.py:425-551) the chunks run over the env-major /
+        time-minor flattening g = n*T + t instead, every chunk step carrying all A agents; the minibatch moments are
+        agent 0's returns / active masks plus the all-agent active sum (4 doubles)."""
         cfg = self.cfg
-        T, B = buf.episode_length, buf.n_rollout_threads * buf.num_agents
+        T, A = buf.episode_length, buf.num_agents
+        B = buf.n_rollout_threads * A
         total, L = T * B, (T if self.naive else cfg.data_chunk_length)
-        if total < L:
+        flat = T * buf.n_rollout_threads if self.joint else total   # flattened samples that are cut into chunks
+        if flat < L:
             raise AssertionError(f"PPO requires the number of processes ({buf.n_rollout_threads}) * episode length ({T}) "
-                                 f"* agents to be greater than or equal to the data chunk length ({L}).")
-        data_chunks = total // L
+                                 f"{'' if self.joint else '* agents '}to be greater than or equal to the data chunk length ({L}).")
+        data_chunks = flat // L
         mbc = data_chunks // self.num_mini_batch
         rows = mbc * L
-        need = int(self._lib.orl_rnn_workspace_floats(rows, self.rnn_stride))   # tape rows + reduction partials
+        tape_rows = rows * A if self.joint else rows   # the JRPO policy tape has one row per agent and chunk step
+        need = int(self._lib.orl_rnn_workspace_floats(tape_rows, self.rnn_stride))   # tape rows + reduction partials
         if self.tape is None or self.tape.numel() < need:
             self.tape = torch.empty(need, dtype=torch.float32, device=self.device)
-        whole = self.num_mini_batch == 1 and rows == total
+        whole = self.num_mini_batch == 1 and rows == flat
         s, Lb = lib.current_stream(), self._lib
-        for _ in range(self.ppo_epoch):
+        for epoch in range(self.ppo_epoch):
             if cfg.parity_mode:
                 perm = torch.randperm(data_chunks).to(self.device, non_blocking=True)   # global CPU generator
                 self.h2d_bytes += data_chunks * 8
@@ -242,8 +273,13 @@ class PPOAlgorithm:
                 perm = torch.randperm(data_chunks, device=self.device)
             for i in range(self.num_mini_batch):
                 ids = perm[i * mbc:(i + 1) * mbc].contiguous()
-                if whole:
+                if whole and not self.joint:
                     mb_stats = buf.gae_stats[5:8]
+                elif whole and epoch > 0:
+                    mb_stats = self.mb_stats   # JRPO, one minibatch of every chunk: the moments of epoch 0 still hold
+                elif self.joint:
+                    mb_stats = self.joint_minibatch_stats(buf, ids, L)
+                    parallel.allreduce_sum_(mb_stats)
                 else:
                     bi = chunk_row_indices(ids, L, T, B)
                     lib.check(Lb.orl_minibatch_stats(lib.ptr(bi), int(rows), lib.ptr(buf.returns), lib.ptr(buf.active_masks),

@@ -29,6 +29,19 @@ def chunk_row_indices(chunk_ids, chunk_length, episode_length, rows):
     return ((f % episode_length) * rows + f // episode_length).contiguous()
 
 
+def chunk_row_indices_v3(chunk_ids, chunk_length, episode_length, n_envs, n_agents, agent0_only=False):
+    """Buffer row indices of the data chunks of `recurrent_generator_v3` (replay_data.py:425-551, the joint-action
+    loss): (T, N, A, ...) is flattened env-major / time-minor (`_cast_v3`, buffers/utils/util.py:99-101), sample
+    g = n*T + t carrying all A agents; chunk c holds g in [c*L, c*L + L).  Step g of agent a is buffer row
+    (g % T)*N*A + (g // T)*A + a.  Ordered (chunk, step, agent); agent0_only keeps agent 0's rows (the critic's
+    `to_single_np`, ppo.py:222-224)."""
+    lane = torch.arange(chunk_length, device=chunk_ids.device)
+    g = (chunk_ids[:, None] * chunk_length + lane[None, :]).reshape(-1, 1)
+    base = (g % episode_length) * (n_envs * n_agents) + (g // episode_length) * n_agents
+    agents = torch.arange(1 if agent0_only else n_agents, device=chunk_ids.device)
+    return (base + agents[None, :]).reshape(-1).contiguous()
+
+
 class ReplayData:
     def __init__(self, cfg, num_agents, obs_space, act_space, data_client=None, episode_length=None, device="cuda:0"):
         T = cfg.episode_length if episode_length is None else episode_length

@@ -682,6 +682,10 @@ extern "C" int orl_ppo_fwdbwd(const OrlPpoArgs* args, void* stream) {
     ORL_CHECK_ARG(args, "args");
     const OrlPpoArgs& a = *args;
     if (int e = check_ppo_args(a)) return e;
+    if (a.flags & ORL_PPO_JOINT_ACTION) {
+        orl::set_last_error("orl_ppo_fwdbwd: ORL_PPO_JOINT_ACTION needs chunked recurrence (orl_rnn_fwdbwd)");
+        return ORL_ERR_UNSUPPORTED;
+    }
     ORL_CHECK_ARG(a.policy_obs && a.critic_obs && a.actions && a.old_log_probs && a.advantages && a.value_preds &&
                       a.returns && a.active_masks && a.gae_stats && a.mb_stats, "null rollout buffer");
     ORL_CHECK_ARG(!(a.flags & ORL_PPO_VALUENORM) || a.vn_state, "vn_state required with VALUENORM");

@@ -5,6 +5,8 @@
 //   OnPolicyDriver.act / add2buffer       openrl/drivers/onpolicy_driver.py:80-152,236-279 (rnn-state carry,
 //                                         zeroing on dones_env)
 //   ReplayData.recurrent_generator        openrl/buffers/replay_data.py:1062-1258 (chunks of L over f=(n*A+a)*T+t)
+//   ReplayData.recurrent_generator_v3     openrl/buffers/replay_data.py:425-551 (JRPO: chunks of L over g=n*T+t, all agents
+//                                         of a step together; joint-action loss ppo.py:254-321)
 //   PPOAlgorithm.ppo_update (BPTT part)   openrl/algorithms/ppo.py:46-458
 //
 // Design (DESIGN.md "recurrent path"): ONE WARP per env (rollout), per row (critic) or per chunk (update) running
@@ -199,11 +201,16 @@ __global__ void __launch_bounds__(W_NT, 1) rnn_critic_warp_kernel(const OrlRnnAr
 }
 
 // ---- update: one warp per C_R chunks; L forward steps (tape), per-step loss, L backward steps ----
-template <bool POLICY, int C_R, int C_NT>
+// JOINT (ORL_PPO_JOINT_ACTION, chunks over g = n*T + t): the policy warp owns ONE chunk and its C_R = A agent rows
+// (tape row (cpos*L + l)*A + a) and takes the joint-action loss once per step; the critic warp runs agent 0's row
+// n*A of each of its C_R chunks.
+template <bool POLICY, int C_R, int C_NT, bool JOINT = false>
 __global__ void __launch_bounds__(C_NT, 1) rnn_chunk_warp_kernel(const OrlRnnArgs a) {
     constexpr int C_WPC = C_NT / 32;
+    constexpr bool JPOL = JOINT && POLICY;   // the warp's rows are the agents of one chunk
     extern __shared__ __align__(16) float smem[];
     const int B = a.n_envs * a.n_agents, T = a.episode_length, L = a.chunk_length;
+    const int rstride = JOINT ? a.n_agents : 1;   // buffer row of flattened sample f (agent r): (f / T) * rstride + r
     const int d = POLICY ? a.obs_dim : a.critic_obs_dim, n = POLICY ? a.n_actions : 1;
     const float* obs = POLICY ? a.policy_obs : a.critic_obs;
     const float* states = POLICY ? a.rnn_states : a.rnn_states_critic;
@@ -214,9 +221,12 @@ __global__ void __launch_bounds__(C_NT, 1) rnn_chunk_warp_kernel(const OrlRnnArg
     float* scr = smem + rw::smem_net_floats() + warp * C_R * rw::SCR;
     float loss0 = 0.f, loss1 = 0.f, loss2 = 0.f;   // identical on every lane; lane 0's copy is reduced
 
-    const double rows_d = a.norm_rows > 0 ? (double)a.norm_rows : (double)a.n_chunks * L;
+    const double rows_d = a.norm_rows > 0 ? (double)a.norm_rows : (double)a.n_chunks * L;   // JOINT: chunk steps
     const float inv_rows = (float)(1.0 / rows_d);
-    const float inv_act = (float)(1.0 / a.mb_stats[2]);
+    const float inv_act = (float)(1.0 / a.mb_stats[2]);   // JOINT: agent 0's active sum
+    // JRPO entropy: mean over all agent rows, or weighted by every agent's active mask (act.py:114-118)
+    const float inv_ent_rows = JPOL ? (float)(1.0 / (rows_d * C_R)) : inv_rows;
+    const float inv_ent_act = JPOL ? (float)(1.0 / a.mb_stats[3]) : inv_act;
     const bool pol_masks = a.flags & ORL_PPO_POLICY_ACTIVE_MASKS, val_masks = a.flags & ORL_PPO_VALUE_ACTIVE_MASKS;
     AdvNorm advn;
     float vn_mean = 0.f, vn_std = 1.f;
@@ -228,17 +238,23 @@ __global__ void __launch_bounds__(C_NT, 1) rnn_chunk_warp_kernel(const OrlRnnArg
         vn_mean = s.mean; vn_std = s.std;
     }
 
-    const long long n_groups = (a.n_chunks + C_R - 1) / C_R;
+    const long long n_groups = JPOL ? a.n_chunks : (a.n_chunks + C_R - 1) / C_R;
     for (long long grp = (long long)blockIdx.x * C_WPC + warp; grp < n_groups; grp += (long long)gridDim.x * C_WPC) {
         long long cpos[C_R], f0[C_R];
+        int agent[C_R];
         bool valid[C_R];
         rw::V2 h[C_R];
 #pragma unroll
         for (int r = 0; r < C_R; ++r) {
-            valid[r] = grp * C_R + r < a.n_chunks;
-            cpos[r] = valid[r] ? grp * C_R + r : grp * C_R;   // a tail slot recomputes chunk 0 of the group (same values, same addresses)
+            if (JPOL) {
+                valid[r] = true; cpos[r] = grp; agent[r] = r;
+            } else {
+                valid[r] = grp * C_R + r < a.n_chunks;
+                cpos[r] = valid[r] ? grp * C_R + r : grp * C_R;   // a tail slot recomputes chunk 0 of the group (same values, same addresses)
+                agent[r] = 0;
+            }
             f0[r] = a.chunk_ids[cpos[r]] * (long long)L;
-            h[r] = rw::ldv(states + ((size_t)(f0[r] % T) * B + (size_t)(f0[r] / T)) * rc::H, lane);
+            h[r] = rw::ldv(states + ((size_t)(f0[r] % T) * B + (size_t)(f0[r] / T) * rstride + agent[r]) * rc::H, lane);
         }
         for (int l = 0; l < L; ++l) {
             rw::V2 x[C_R], h2[C_R];
@@ -247,52 +263,93 @@ __global__ void __launch_bounds__(C_NT, 1) rnn_chunk_warp_kernel(const OrlRnnArg
             size_t bi[C_R];
 #pragma unroll
             for (int r = 0; r < C_R; ++r) {
-                const long long f = f0[r] + l, row = f / T, t = f % T;
+                const long long f = f0[r] + l, row = (f / T) * rstride + agent[r], t = f % T;
                 bi[r] = (size_t)t * B + row;
                 const float* ob = obs + bi[r] * d;
                 x[r] = rw::V2{lane < d ? ob[lane] : 0.f, lane + 32 < d ? ob[lane + 32] : 0.f};
                 mk[r] = a.masks[bi[r]];
-                tape[r] = a.tape + ((size_t)cpos[r] * L + l) * rw::TAPE_W;
+                tape[r] = a.tape + (JPOL ? ((size_t)cpos[r] * L + l) * C_R + r : (size_t)cpos[r] * L + l) * rw::TAPE_W;
             }
             rw::step_forward<C_R>(W, scr, d, n, a.activation_id, x, h, mk, h2, out, tape, lane);
+            if constexpr (JPOL) {
+                // joint log-prob of the step: register sum over the warp's agent rows, in agent order (ppo.py:284-300)
+                float joint = 0.f, old_joint = 0.f;
 #pragma unroll
-            for (int r = 0; r < C_R; ++r) {
-                h[r] = h2[r];
-                float dl[MAX_OUT];
-#pragma unroll
-                for (int j = 0; j < MAX_OUT; ++j) dl[j] = 0.f;
-                const float active = a.active_masks[bi[r]];
-                const float keep = valid[r] ? 1.f : 0.f;
-                if (POLICY) {
+                for (int r = 0; r < C_R; ++r) {
+                    h[r] = h2[r];
                     float nl[MAX_OUT], pr[MAX_OUT];
                     log_softmax_n(out[r], n, nl, pr);
                     const int act = (int)a.actions[bi[r]];
                     float lp = nl[0];
 #pragma unroll
                     for (int j = 1; j < MAX_OUT; ++j) if (j == act) lp = nl[j];
-                    const float adv = apply_adv_norm(advn, a.advantages[bi[r]]);
-                    const PgTerm pg = pg_term(lp, a.action_log_probs[bi[r]], adv, a.clip_param, a.flags, a.dual_clip_coeff);
-                    const float wrow = pol_masks ? active * inv_act : inv_rows;
+                    joint += lp;
+                    old_joint += a.action_log_probs[bi[r]];
+                }
+                const float adv = apply_adv_norm(advn, a.advantages[bi[0]]);
+                const PgTerm pg = pg_term(joint, old_joint, adv, a.clip_param, a.flags, a.dual_clip_coeff);
+                const float wrow = pol_masks ? a.active_masks[bi[0]] * inv_act : inv_rows;
+                loss0 += pg.loss * wrow; loss2 += pg.ratio;
+                const float dlp = pg.dlogp * wrow;   // every agent row of the step receives the same dL/dlogp_joint
+#pragma unroll
+                for (int r = 0; r < C_R; ++r) {
+                    float nl[MAX_OUT], pr[MAX_OUT], dl[MAX_OUT];
+                    log_softmax_n(out[r], n, nl, pr);
+                    const int act = (int)a.actions[bi[r]];
+                    const float went = pol_masks ? a.active_masks[bi[r]] * inv_ent_act : inv_ent_rows;
                     float ent = 0.f;
 #pragma unroll
                     for (int j = 0; j < MAX_OUT; ++j) if (j < n) ent -= pr[j] * nl[j];
-                    loss0 += keep * pg.loss * wrow; loss1 += keep * ent * wrow; loss2 += keep * pg.ratio;
-                    const float dlp = pg.dlogp * wrow, went = a.entropy_coef * wrow;
+                    loss1 += ent * went;
+                    const float wec = a.entropy_coef * went;
 #pragma unroll
                     for (int j = 0; j < MAX_OUT; ++j)
-                        if (j < n) dl[j] = dlp * ((j == act ? 1.f : 0.f) - pr[j]) + went * pr[j] * (nl[j] + ent);
-                } else {
-                    const float ret = a.returns[bi[r]];
-                    const float target = (a.flags & ORL_PPO_VALUENORM) ? (ret - vn_mean) / vn_std : ret;
-                    const ValueTerm vt = value_term(out[r][0], a.value_preds[bi[r]], target, a.clip_param, a.huber_delta, a.flags);
-                    const float wrow = val_masks ? active * inv_act : inv_rows;
-                    loss0 += keep * vt.loss * wrow;
-                    dl[0] = a.value_loss_coef * wrow * vt.dv;
-                }
-                float mine = 0.f;   // lane m < 8 stores dL/dout[m]
+                        dl[j] = j < n ? dlp * ((j == act ? 1.f : 0.f) - pr[j]) + wec * pr[j] * (nl[j] + ent) : 0.f;
+                    float mine = 0.f;   // lane m < 8 stores dL/dout[m]
 #pragma unroll
-                for (int j = 0; j < MAX_OUT; ++j) if (lane == j) mine = dl[j];
-                if (lane < MAX_OUT) tape[r][rc::TP_DLOG + lane] = mine;
+                    for (int j = 0; j < MAX_OUT; ++j) if (lane == j) mine = dl[j];
+                    if (lane < MAX_OUT) tape[r][rc::TP_DLOG + lane] = mine;
+                }
+            } else {
+#pragma unroll
+                for (int r = 0; r < C_R; ++r) {
+                    h[r] = h2[r];
+                    float dl[MAX_OUT];
+#pragma unroll
+                    for (int j = 0; j < MAX_OUT; ++j) dl[j] = 0.f;
+                    const float active = a.active_masks[bi[r]];
+                    const float keep = valid[r] ? 1.f : 0.f;
+                    if (POLICY) {
+                        float nl[MAX_OUT], pr[MAX_OUT];
+                        log_softmax_n(out[r], n, nl, pr);
+                        const int act = (int)a.actions[bi[r]];
+                        float lp = nl[0];
+#pragma unroll
+                        for (int j = 1; j < MAX_OUT; ++j) if (j == act) lp = nl[j];
+                        const float adv = apply_adv_norm(advn, a.advantages[bi[r]]);
+                        const PgTerm pg = pg_term(lp, a.action_log_probs[bi[r]], adv, a.clip_param, a.flags, a.dual_clip_coeff);
+                        const float wrow = pol_masks ? active * inv_act : inv_rows;
+                        float ent = 0.f;
+#pragma unroll
+                        for (int j = 0; j < MAX_OUT; ++j) if (j < n) ent -= pr[j] * nl[j];
+                        loss0 += keep * pg.loss * wrow; loss1 += keep * ent * wrow; loss2 += keep * pg.ratio;
+                        const float dlp = pg.dlogp * wrow, went = a.entropy_coef * wrow;
+#pragma unroll
+                        for (int j = 0; j < MAX_OUT; ++j)
+                            if (j < n) dl[j] = dlp * ((j == act ? 1.f : 0.f) - pr[j]) + went * pr[j] * (nl[j] + ent);
+                    } else {
+                        const float ret = a.returns[bi[r]];
+                        const float target = (a.flags & ORL_PPO_VALUENORM) ? (ret - vn_mean) / vn_std : ret;
+                        const ValueTerm vt = value_term(out[r][0], a.value_preds[bi[r]], target, a.clip_param, a.huber_delta, a.flags);
+                        const float wrow = val_masks ? active * inv_act : inv_rows;
+                        loss0 += keep * vt.loss * wrow;
+                        dl[0] = a.value_loss_coef * wrow * vt.dv;
+                    }
+                    float mine = 0.f;   // lane m < 8 stores dL/dout[m]
+#pragma unroll
+                    for (int j = 0; j < MAX_OUT; ++j) if (lane == j) mine = dl[j];
+                    if (lane < MAX_OUT) tape[r][rc::TP_DLOG + lane] = mine;
+                }
             }
         }
         __syncwarp();   // tape scalars (lane 0) and dL/dout (lanes < 8) are read by every lane below
@@ -302,7 +359,8 @@ __global__ void __launch_bounds__(C_NT, 1) rnn_chunk_warp_kernel(const OrlRnnArg
         for (int l = L - 1; l >= 0; --l) {
             float* tape[C_R];
 #pragma unroll
-            for (int r = 0; r < C_R; ++r) tape[r] = a.tape + ((size_t)cpos[r] * L + l) * rw::TAPE_W;
+            for (int r = 0; r < C_R; ++r)
+                tape[r] = a.tape + (JPOL ? ((size_t)cpos[r] * L + l) * C_R + r : (size_t)cpos[r] * L + l) * rw::TAPE_W;
             rw::step_backward<C_R>(W, scr, n, a.activation_id, tape, dh, lane);
         }
     }
@@ -515,6 +573,20 @@ int warp_grid(long long units) {   // persistent CTAs: one per SM, never more th
     return (int)std::max(1LL, std::min<long long>(need, orl::sm_count()));
 }
 
+constexpr int JOINT_MAX_AGENTS = 4;   // JRPO policy warps hold one chunk's A agent rows (C_R = A)
+static_assert(w_smem(JOINT_MAX_AGENTS) <= 227 * 1024, "JRPO policy weights + scratch must fit one CTA per SM");
+
+// one persistent warp kernel launch over `units` warp work items (chunk groups)
+template <bool POLICY, int C_R, bool JOINT>
+int launch_chunk(const OrlRnnArgs& a, long long units, cudaStream_t st) {
+    auto k = rnn_chunk_warp_kernel<POLICY, C_R, W_NT, JOINT>;
+    if (int e = warp_kernel_prepare(k, w_smem(C_R), POLICY ? "smem attr (rnn chunk policy)" : "smem attr (rnn chunk critic)")) return e;
+    k<<<warp_grid(units), W_NT, w_smem(C_R), st>>>(a);
+    return 0;
+}
+template <int A>
+int launch_joint_policy(const OrlRnnArgs& a, cudaStream_t st) { return launch_chunk<true, A, true>(a, a.n_chunks, st); }
+
 int check_common(const OrlRnnArgs& a) {
     ORL_CHECK_ARG(a.n_envs > 0 && a.n_agents > 0 && a.episode_length > 0, "n_envs / n_agents / episode_length");
     ORL_CHECK_ARG(a.obs_dim > 0 && a.obs_dim <= rc::MAXD && a.critic_obs_dim > 0 && a.critic_obs_dim <= rc::MAXD, "obs dims (<= 64)");
@@ -600,24 +672,41 @@ int orl_rnn_fwdbwd(const OrlRnnArgs* ap, void* stream) {
     ORL_CHECK_ARG(a.grads_stride >= rc::rnn_offsets(a.obs_dim, a.n_actions).total &&
                       a.grads_stride >= rc::rnn_offsets(a.critic_obs_dim, 1).total, "grads_stride");
     if (a.flags & ORL_PPO_VALUENORM) { ORL_CHECK_ARG(a.vn_state, "vn_state"); }
+    const bool joint = a.flags & ORL_PPO_JOINT_ACTION;
+    if (joint && a.n_agents > JOINT_MAX_AGENTS) {
+        orl::set_last_error("orl_rnn_fwdbwd: ORL_PPO_JOINT_ACTION is built for n_agents <= %d (got %d)", JOINT_MAX_AGENTS, a.n_agents);
+        return ORL_ERR_UNSUPPORTED;
+    }
     cudaStream_t st = (cudaStream_t)stream;
     int e = orl::check_cuda(cudaMemsetAsync(a.loss_acc, 0, 8 * sizeof(float), st), "memset loss_acc");
     if (e) return e;
-    const long long rows = a.n_chunks * a.chunk_length;
-    const int rb = ws_row_blocks(rows);
-    float* partials = a.tape + ws_tape_floats(rows);
+    // tape rows per net: n_chunks*L chunk steps, times A policy rows per step with the joint-action loss
+    const long long steps = a.n_chunks * a.chunk_length;
+    const long long net_rows[2] = {joint ? steps * a.n_agents : steps, steps};
+    float* partials = a.tape + ws_tape_floats(net_rows[0]);
     // two chunks per warp: every weight read from shared memory feeds two rows (four per warp with 8 warps / CTA
-    // measured 12 % slower on B200: profiles/r1_gru_perf.md)
+    // measured 12 % slower on B200: profiles/r1_gru_perf.md).  JRPO policy: one chunk per warp, its A agent rows.
     constexpr int C_R = 2;
     if ((e = orl::check_cuda(cudaFuncSetAttribute(tape_gemm_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TR_SMEM),
                              "smem attr (tape gemm)"))) return e;
-    if ((e = warp_kernel_prepare(rnn_chunk_warp_kernel<true, C_R, W_NT>, w_smem(C_R), "smem attr (rnn chunk policy)"))) return e;
-    if ((e = warp_kernel_prepare(rnn_chunk_warp_kernel<false, C_R, W_NT>, w_smem(C_R), "smem attr (rnn chunk critic)"))) return e;
-    const int cgrid = warp_grid((a.n_chunks + C_R - 1) / C_R);
     for (int net = 0; net < 2; ++net) {
         const int d = net == 0 ? a.obs_dim : a.critic_obs_dim, n = net == 0 ? a.n_actions : 1;
-        if (net == 0) rnn_chunk_warp_kernel<true, C_R, W_NT><<<cgrid, W_NT, w_smem(C_R), st>>>(a);
-        else rnn_chunk_warp_kernel<false, C_R, W_NT><<<cgrid, W_NT, w_smem(C_R), st>>>(a);
+        if (net == 0 && joint) {
+            switch (a.n_agents) {
+                case 1: e = launch_joint_policy<1>(a, st); break;
+                case 2: e = launch_joint_policy<2>(a, st); break;
+                case 3: e = launch_joint_policy<3>(a, st); break;
+                default: e = launch_joint_policy<4>(a, st); break;
+            }
+        } else if (net == 0) {
+            e = launch_chunk<true, C_R, false>(a, (a.n_chunks + C_R - 1) / C_R, st);
+        } else {
+            e = joint ? launch_chunk<false, C_R, true>(a, (a.n_chunks + C_R - 1) / C_R, st)
+                      : launch_chunk<false, C_R, false>(a, (a.n_chunks + C_R - 1) / C_R, st);
+        }
+        if (e) return e;
+        const long long rows = net_rows[net];
+        const int rb = ws_row_blocks(rows);
         const TapeJobs jobs = make_jobs(d, n);
         tape_gemm_kernel<<<dim3(rb, jobs.n_gemm), TR_NT, TR_SMEM, st>>>(a.tape, rows, jobs, partials, a.grads_stride);
         tape_colsum_kernel<<<dim3(rb, jobs.n_col), rc::G3, 0, st>>>(a.tape, rows, jobs, partials, a.grads_stride);

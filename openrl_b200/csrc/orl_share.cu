@@ -369,6 +369,10 @@ int orl_share_fwdbwd(const OrlPpoArgs* ap, void* stream) {
     ORL_CHECK_ARG(a.policy_params && a.partials && a.folded && a.grads && a.policy_obs && a.actions && a.old_log_probs && a.advantages &&
                       a.value_preds && a.returns && a.active_masks && a.gae_stats && a.mb_stats, "null buffer");
     ORL_CHECK_ARG(a.head_kind == ORL_HEAD_CATEGORICAL, "the shared-model kernels are built for Discrete action spaces");
+    if (a.flags & ORL_PPO_JOINT_ACTION) {
+        orl::set_last_error("orl_share_fwdbwd: ORL_PPO_JOINT_ACTION needs chunked recurrence (orl_rnn_fwdbwd)");
+        return ORL_ERR_UNSUPPORTED;
+    }
     cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
     float* tape = a.partials;
     const long long rows = a.batch_rows;

@@ -230,3 +230,4 @@ PPO_HUBER, PPO_CLIP_VALUE, PPO_VALUE_ACTIVE_MASKS, PPO_POLICY_ACTIVE_MASKS = 1, 
 PPO_VALUENORM, PPO_ADV_NORMALIZE, PPO_MAX_GRAD_NORM, PPO_TENSORCORE = 16, 32, 64, 128
 PPO_TF32 = PPO_TENSORCORE   # round-1 name
 PPO_A2C, PPO_DUAL_CLIP = 256, 512
+PPO_JOINT_ACTION = 1024   # cfg.use_joint_action_loss (JRPO): chunked recurrent update only
